@@ -4,6 +4,7 @@
     python bench.py --gpus 1 --steps K --warmup W                  # this repo's CUDA path
     torchrun ... bench.py --gpus N ...                             # one rank per GPU, time shards + halo
     python bench.py --impl reference ...                           # the reference's CPU path (oracle port)
+    python bench.py ... --dump-outputs DIR                         # + DIR/<name>.npy of the last timed step
 
 A "step" is one pass of the hot path over the whole workload: `--frames` synthetic 1920x1080
 BGR24 frames per GPU (default 10 000 = 62.2 GB, far larger than L2, so no flush is needed),
@@ -28,12 +29,20 @@ import numpy as np  # noqa: E402
 
 METRIC = "frames/sec scored (1080p, ContentDetector)"
 UNIT = "frames/s"
+DUMP_BYTES = 60 * 2**20  # --dump-outputs: larger outputs are written as a fixed, seeded sample of frames
+
+
+def _positive_int(text: str) -> int:
+    v = int(text)
+    if v < 1:
+        raise argparse.ArgumentTypeError(f"must be >= 1, got {v}")
+    return v
 
 
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=_positive_int, default=10, help="timed steps")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--frames", type=int, default=10000, help="frames per GPU per step")
@@ -63,7 +72,27 @@ def parse_args():
     ap.add_argument("--sweep-cells", default="640x360,1280x720,1920x1080,3840x2160:1000,10000,100000")
     ap.add_argument("--auto-downscale", action="store_true",
                     help="score at SceneManager's default auto-downscaled size (256 px wide) instead of full resolution")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the per-frame arrays the last timed step computed as DIR/<name>.npy (float32/float64; "
+                         f"a seeded sample of frames above {DUMP_BYTES >> 20} MiB; _rank<r> suffix with several GPUs)")
+    args = ap.parse_args()
+    if args.dump_outputs and (args.sweep or args.impl != "ours"):
+        ap.error("--dump-outputs needs --impl ours and no --sweep")
+    return args
+
+
+def dump_outputs(path: str, arrays: dict, suffix: str = "") -> None:
+    """Per-frame result arrays -> path/<name><suffix>.npy.  Above DUMP_BYTES, the same seeded sample of frames
+    is kept from every array and its frame indices are written as frame_index<suffix>.npy."""
+    os.makedirs(path, exist_ok=True)
+    n = len(next(iter(arrays.values())))
+    per_frame = sum(a.nbytes // n for a in arrays.values())
+    if per_frame * n > DUMP_BYTES:
+        keep = np.sort(np.random.default_rng(0).choice(n, DUMP_BYTES // (per_frame + 8), replace=False))
+        arrays = {k: a[keep] for k, a in arrays.items()}
+        arrays["frame_index"] = keep.astype(np.float64)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, f"{name}{suffix}.npy"), a)
 
 
 # ------------------------------------------------------------------------------------------
@@ -462,6 +491,18 @@ def run_ours(args):
     sampler.window = (t0, t0 + wall)
     clocks = sampler.stop() if rank == 0 else None
     launches = lib.psd_launch_count() - launches0
+    if args.dump_outputs:
+        # what a caller of the timed path receives from its last step: the per-frame metric, and for the
+        # content detectors the four components and the >= threshold flags (adaptive: the ratio instead)
+        name = {"threshold": "average_rgb", "histogram": "hist_diff", "hash": "hash_dist"}.get(args.detector, "content_val")
+        out = {name: d_val.cpu().numpy()}
+        if args.detector in ("content", "content_edges", "adaptive"):
+            out["components"] = d_comp.view(N, 4).cpu().numpy()
+        if args.detector == "adaptive":
+            out["adaptive_ratio"] = d_ratio.cpu().numpy()
+        elif args.detector in ("content", "content_edges"):
+            out["above_threshold"] = d_flag.cpu().numpy().astype(np.float32)
+        dump_outputs(args.dump_outputs, out, f"_rank{rank}" if world > 1 else "")
     # device time per step (CUDA events on the engine's compute stream) and wall time; max over ranks
     t = torch.tensor([ev_ms_total / args.steps, 1000.0 * wall / args.steps], dtype=torch.float64, device=f"cuda:{dev}")
     if world > 1:
@@ -704,7 +745,7 @@ def main():
                 a.width, a.height = (int(v) for v in size.split("x"))
                 a.frames, a.scaling = int(total), "strong"
                 a.no_e2e = a.no_cpu = True
-                a.steps, a.warmup = min(args.steps, 5), 3
+                a.steps, a.warmup = args.steps, args.warmup
                 a.parity_frames = 8
                 run_ours(a)
     else:

@@ -5,11 +5,10 @@ When the real `scenedetect` package is importable, its own `SceneDetector`, `Fla
 common.py:191-811, stats_manager.py:85-314) - the detectors in this package then subclass the
 reference's ABC and drop straight into the reference `SceneManager`.
 
-On a box without the reference (the GPU test box has no /root/reference) the minimal,
-independently written equivalents below are used instead.  They implement only the
-constant-frame-rate, frame-number-backed behaviour the hot path needs, with the same
-observable semantics (comparison/rounding rules, CSV layout), and are pinned against the real
-classes by tests/test_compat_vs_reference.py whenever the reference is present.
+Where `scenedetect` is not importable, the minimal, independently written equivalents below
+are used instead.  They implement only the constant-frame-rate, frame-number-backed behaviour
+the hot path needs, with the same observable semantics (comparison/rounding rules, CSV layout),
+and are pinned against the real classes' recorded behaviour by tests/test_compat_vs_reference.py.
 """
 
 from __future__ import annotations
